@@ -3,6 +3,7 @@
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--config fused|lm_only|amis|dense|train]   # our arm
     python bench.py --impl reference [--gpus N] [--steps K] [--config ...]                          # CPU arm
+    python bench.py ... --dump-outputs DIR     # also write what the last timed step returned, DIR/<name>.npy
 
 Default = the headline metric: PnP objects/sec at (B = 4096 per GPU, N = 512, M = 512), BASELINE.json configs #3 / #5's
 shape.  One "step" = one pass of the hot path over one batch of synthetic correspondence sets through ONE C-ABI call
@@ -22,6 +23,12 @@ BASELINE.json's #2 (LM only, B = 1024), #3 (B = 1024), #4 (dense 64 x 64 coordin
   cpu_baseline   the UNMODIFIED reference layer (oracle/_ref staged by oracle/stage_ref.py + oracle/pyro_shim) -- or the
              oracle port when it has not been staged -- on all host cores (one worker process per 4 cores, the objects
              are independent), bounded sample; rank 0, N = 1 only.
+
+--dump-outputs DIR writes, after the timed steps, the arrays the last timed step returned as DIR/<name>.npy (float32;
+at most DUMP_MAX_BYTES, else a fixed, seeded sample of objects); the training config adds dL/dx2d and dL/dw2d, which
+the step leaves in the leaves' .grad.  Inputs and seeds depend only on the arguments, so two builds can be compared
+output for output.  With N > 1 only rank 0's own objects are written, not the gathered full batch: a deliberate limit
+(the gathered pose_opt / logw rows of rank 0 hold the same values).
 """
 import argparse
 import json
@@ -67,6 +74,7 @@ WARM_SECONDS = 0.5            # minimum duration of back-to-back warm-up launche
 # puts the pages on the GPU's NUMA node; a remote node costs upload bandwidth)
 E2E_NUMA = os.environ.get("EPNP_E2E_NUMA", "1") == "1"
 L2_BYTES = 126e6
+DUMP_MAX_BYTES = 64_000_000   # --dump-outputs writes at most this many bytes, .npy headers included
 
 
 class gpu_local_cpus:
@@ -267,6 +275,36 @@ def rotating_sets(cfg):
     return max(2, min(16, int(math.ceil(1.15 * L2_BYTES / set_bytes)) + 1)), set_bytes
 
 
+def npy_bytes(a):
+    """Size of the .npy file np.save writes for `a`: header + data."""
+    import io
+    import numpy as np
+    buf = io.BytesIO()
+    np.lib.format.write_array_header_1_0(buf, np.lib.format.header_data_from_array_1_0(a))
+    return buf.tell() + a.nbytes
+
+
+def host_outputs(out, n_obj):
+    """--dump-outputs: the arrays of one step's result dict (absent ones skipped) as float32 / float64 numpy arrays.
+    When their .npy files would come to more than DUMP_MAX_BYTES, every per-object array (leading dimension n_obj) keeps
+    the same fixed, seeded sample of objects, in object order: the largest sample that fits."""
+    import numpy as np
+    arrs = {}
+    for name, t in out.items():
+        if t is not None:
+            a = t.detach().cpu().numpy()
+            arrs[name] = a if a.dtype in (np.float32, np.float64) else a.astype(np.float32)
+    per_obj = [name for name, a in arrs.items() if a.ndim and a.shape[0] == n_obj]
+    total = sum(npy_bytes(a) for a in arrs.values())     # a sample's headers are no longer than these
+    if total > DUMP_MAX_BYTES:
+        obj_bytes = sum(arrs[name].nbytes for name in per_obj) // n_obj
+        keep = (DUMP_MAX_BYTES - (total - obj_bytes * n_obj)) // obj_bytes
+        idx = np.sort(np.random.default_rng(0).choice(n_obj, size=keep, replace=False))
+        for name in per_obj:
+            arrs[name] = arrs[name][idx]
+    return arrs
+
+
 def config_block(args, cfg, world):
     """The `config` object of the JSON line -- the SAME for both arms (`--impl ours` / `--impl reference`): it names the
     workload; what is specific to how the CPU arm samples it goes into that arm's `cpu_baseline.sample`."""
@@ -286,15 +324,15 @@ def config_block(args, cfg, world):
 def run_reference_arm(args, cfg, rank):
     if rank != 0:
         return
-    # the whole arm is bounded to about 2.5 minutes whatever K and W are
-    per_step = max(1.0, min(20.0, 140.0 / max(1, args.steps + args.warmup)))
-    steps = args.steps if (args.steps + args.warmup) * per_step <= 150 else max(1, int(150 / per_step) - args.warmup)
+    # exactly K timed steps; the arm aims at about 2.5 minutes whatever K and W are, so a step's slice shrinks as K grows
+    # (a worker's slice still runs at least one whole pass, so at large K the arm takes K + W passes)
+    per_step = min(20.0, 140.0 / (args.steps + args.warmup))
     t0 = time.perf_counter()
-    rates, cores, kind, sample = cpu_reference_rates(cfg, steps, args.warmup, per_step)
+    rates, cores, kind, sample = cpu_reference_rates(cfg, args.steps, args.warmup, per_step)
     el = time.perf_counter() - t0
     value = statistics.mean(rates)
     line = {"impl": "reference", "metric": cfg["metric"], "value": value, "unit": "objects/s", "n_gpus": args.gpus,
-            "steps": args.steps, "steps_run": steps, "warmup": args.warmup, "ms_per_step": 1e3 * per_step,
+            "steps": args.steps, "warmup": args.warmup, "ms_per_step": 1e3 * per_step,
             "higher_is_better": True, "scaling": "weak", "vs_baseline": None, "dtype": "f32", "data": "synthetic",
             "config": config_block(args, cfg, int(os.environ.get("WORLD_SIZE", "1"))),
             "cpu_baseline": {"value": value, "unit": "objects/s", "cores": cores, "kind": kind, "sample": sample,
@@ -324,7 +362,12 @@ def main():
                          "so the next batch's LM kernel and first AMIS CTAs fill the SMs the previous batch's last, partial wave "
                          "of CTAs leaves idle (measured +4.4 %% at one GPU); 1 = strictly one batch at a time")
     ap.add_argument("--batch", type=int, default=0, help="objects per GPU (default: the config's)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the arrays the last timed step returned as DIR/<name>.npy, so that "
+                         "two builds can be compared output for output on identical inputs (N > 1: rank 0's own objects only)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     cfg = dict(CONFIGS[args.config])
     if args.batch > 0:
         cfg["B"] = args.batch
@@ -397,8 +440,11 @@ def main():
             x3d.grad = x2d.grad = w2d.grad = None
             cost_fun = AdaptiveHuberPnPCost(relative_delta=cfg["rel_delta"])
             cost_fun.set_param(x2d.detach(), w2d)
+            # the AMIS seed follows the step index, as in solve(): without it each call draws one from torch's generator,
+            # and the time-bounded warm-up would leave the timed steps on different seeds from run to run
             _, _, _, _, logw, cost_tgt = layer.monte_carlo_forward(x3d, x2d, w2d, d["camera"], cost_fun,
-                                                                   pose_init=d["pose_gt"], force_init_solve=False)
+                                                                   pose_init=d["pose_gt"], force_init_solve=False,
+                                                                   amis_seed=1234 + i)
             loss = loss_fn(logw, cost_tgt, 1.0)
             loss.backward()
             return {"loss": loss.detach(), "gx3d": x3d.grad}
@@ -526,6 +572,15 @@ def main():
     wall1 = time.time()
     timing[0] = False
     total_ms = t_begin.elapsed_time(t_end)
+    dump = None
+    if args.dump_outputs and rank == 0:
+        last = out
+        if kind == "train":
+            # a caller of the training step receives all three gradients; train() returns only the loss and dL/dx3d,
+            # which is what the end-to-end section downloads
+            _, x2d, w2d = sets[(args.steps - 1) % n_sets]["leaf"]
+            last = dict(out, gx2d=x2d.grad, gw2d=w2d.grad)
+        dump = host_outputs(last, Bg)
     clocks = sampler.stop(wall0, wall1) if rank == 0 else None
     # the solve's launches inside the loop (first 64 steps): their own duration, and the gap to the next step's launches
     in_loop = None
@@ -681,6 +736,11 @@ def main():
                 line["cpu_baseline"] = {"value": rates[0], "unit": "objects/s", "cores": cores, "kind": ckind, "sample": sample}
             except Exception as ex:                            # noqa: BLE001
                 line["cpu_baseline"] = {"value": None, "error": repr(ex)}
+        if dump is not None:
+            import numpy as np
+            os.makedirs(args.dump_outputs, exist_ok=True)
+            for name, a in dump.items():
+                np.save(os.path.join(args.dump_outputs, name + ".npy"), a)
         print(json.dumps(line), flush=True)
     if world > 1:
         dist.destroy_process_group()

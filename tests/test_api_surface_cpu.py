@@ -1,63 +1,19 @@
 """Drop-in check by introspection: every public function, class, method and static method of the six reference modules
-on the path (epropnp.epropnp, .levenberg_marquardt, .camera, .cost_fun, .common, .distributions) exists under the same
-name in the package, and every parameter of the reference signature is present in ours, in the same order, with the
-same default (ours may append optional keyword arguments).  Needs the reference checkout (/root/reference: present in
-the build container, absent on the GPU box) and the pyro shim; skipped where the reference is not available."""
-import importlib
-import inspect
+(epropnp.epropnp, .levenberg_marquardt, .camera, .cost_fun, .common, .distributions) exists under the same name in the
+package, and every parameter of the reference signature is present in ours, in the same order, with the same default
+(ours may append optional keyword arguments).  The reference surface is tests/golden/api_surface.json, recorded from the
+unmodified reference package by oracle/api_surface.py."""
+import json
 import os
-import subprocess
-import sys
-
-import pytest
 
 from conftest import ROOT
-
-MODULES = ("epropnp.epropnp", "epropnp.levenberg_marquardt", "epropnp.camera", "epropnp.cost_fun", "epropnp.common",
-           "epropnp.distributions")
-REFERENCE = "/root/reference"
-
-_DUMP = r'''
-import importlib, inspect, json, sys
-def params(f):
-    try:
-        return [[p.name, p.kind.name, None if p.default is inspect.Parameter.empty else repr(p.default)]
-                for p in inspect.signature(f).parameters.values()]
-    except (TypeError, ValueError):
-        return None
-out = {}
-for m in sys.argv[2:]:
-    mod = importlib.import_module(m)
-    for n, o in vars(mod).items():
-        if n.startswith('_'):
-            continue
-        own = getattr(o, '__module__', None) == m
-        if inspect.isclass(o) and (own or sys.argv[1] == 'all'):
-            for kls in (o.__mro__ if sys.argv[1] == 'all' else (o,)):
-                for mn, mo in vars(kls).items():
-                    if mn.startswith('__') and mn != '__init__':
-                        continue
-                    f = mo.__func__ if isinstance(mo, (staticmethod, classmethod)) else mo
-                    if callable(f):
-                        out.setdefault(f'{m}:{n}.{mn}', params(f))
-        elif callable(o) and not inspect.isclass(o) and (own or sys.argv[1] == 'all'):
-            out[f'{m}:{n}'] = params(o)
-print(json.dumps(out))
-'''
+from oracle.api_surface import GOLDEN, surface
 
 
-def _surface(paths, mode):
-    env = dict(os.environ, PYTHONPATH=os.pathsep.join(paths))
-    r = subprocess.run([sys.executable, "-c", _DUMP, mode, *MODULES], capture_output=True, text=True, env=env, timeout=300)
-    assert r.returncode == 0, r.stderr[-2000:]
-    import json
-    return json.loads(r.stdout.strip().splitlines()[-1])
-
-
-@pytest.mark.skipif(not os.path.isdir(os.path.join(REFERENCE, "epropnp")), reason="reference checkout not present")
 def test_every_public_name_and_parameter_of_the_reference_exists_here():
-    ref = _surface([os.path.join(ROOT, "oracle", "pyro_shim"), REFERENCE], "own")
-    ours = _surface([os.path.join(ROOT, "epro-pnp_b200"), ROOT], "all")
+    with open(GOLDEN) as f:
+        ref = json.load(f)
+    ours = surface([os.path.join(ROOT, "epro-pnp_b200"), ROOT], "all")
     assert len(ref) > 60
     missing = sorted(k for k in ref if k not in ours)
     assert not missing, missing

@@ -88,6 +88,56 @@ def test_bench_loop_runs_and_prints_the_contract_line(monkeypatch, capsys, argv,
         assert set(e["step_interval_ms"]) == {"min", "median", "max"}
 
 
+def dump_outputs(monkeypatch, capsys, out_dir, argv, **module_overrides):
+    import numpy as np
+    run_bench(monkeypatch, capsys, argv + ["--dump-outputs", str(out_dir)], **module_overrides)
+    return {p.stem: np.load(p) for p in sorted(out_dir.glob("*.npy"))}
+
+
+@pytest.mark.parametrize("config", ["fused", "train"])
+def test_dump_outputs_is_the_last_timed_step(monkeypatch, capsys, tmp_path, config):
+    """--dump-outputs writes what the last timed step returned, in float32 / float64: the same arguments give the same
+    arrays (seeded inputs, AMIS seed = step index), and one more timed step gives a different last step."""
+    import numpy as np
+    argv = ["--config", config, "--no-e2e"]
+    a = dump_outputs(monkeypatch, capsys, tmp_path / "a", argv)
+    b = dump_outputs(monkeypatch, capsys, tmp_path / "b", argv)
+    c = dump_outputs(monkeypatch, capsys, tmp_path / "c", argv + ["--steps", "4"])
+    grads = ("gx3d", "gx2d", "gw2d")
+    assert set(a) == ({"loss", *grads} if config == "train" else {"pose_opt", "pose_cov", "cost", "pose_samples", "logw"})
+    for name, arr in a.items():
+        assert arr.dtype in (np.float32, np.float64) and np.isfinite(arr).all(), name
+        assert np.array_equal(arr, b[name]), name
+    for name in (grads if config == "train" else ("logw",)):
+        assert np.abs(a[name]).max() > 0 and not np.array_equal(a[name], c[name]), name
+
+
+def test_dump_outputs_samples_the_same_objects_of_every_array_above_the_cap(monkeypatch, capsys, tmp_path):
+    import numpy as np
+    argv = ["--batch", "8", "--no-e2e"]
+    full = dump_outputs(monkeypatch, capsys, tmp_path / "full", argv)
+    cap = sum(p.stat().st_size for p in (tmp_path / "full").glob("*.npy")) // 2
+    part = dump_outputs(monkeypatch, capsys, tmp_path / "part", argv, DUMP_MAX_BYTES=cap)
+    assert set(part) == set(full) and sum(p.stat().st_size for p in (tmp_path / "part").glob("*.npy")) <= cap
+    keep = part["pose_opt"].shape[0]
+    assert 0 < keep < 8
+    idx = np.sort(np.random.default_rng(0).choice(8, size=keep, replace=False))
+    for name, arr in part.items():
+        assert np.array_equal(arr, full[name][idx]), name
+
+
+def test_reference_arm_times_exactly_the_requested_steps(monkeypatch, capsys):
+    """--impl reference runs K timed steps however large K is; only the length of a step's slice adapts."""
+    import bench
+    asked = []
+    monkeypatch.setattr(bench, "cpu_reference_rates",
+                        lambda cfg, steps, warmup, per_step: asked.append((steps, warmup)) or ([10.0] * steps, 8, "port", "stub"))
+    monkeypatch.setattr(sys, "argv", ["bench.py", "--impl", "reference", "--steps", "400", "--warmup", "3"])
+    bench.main()
+    line = json.loads([l for l in capsys.readouterr().out.splitlines() if l.startswith("{")][-1])
+    assert asked == [(400, 3)] and line["steps"] == 400
+
+
 @pytest.mark.parametrize("argv", [[], ["--config", "dense"], ["--streams", "1"]])
 def test_both_arms_name_the_same_config(monkeypatch, capsys, argv):
     """`--impl reference` must report the workload of `--impl ours` word for word (the driver pairs the two lines by

@@ -10,6 +10,7 @@
 //                                    4 points per thread between block barriers (DESIGN.md section 4).
 //   cost_kernel, evaluate_full_kernel, rslm_draw_kernel, rslm_kernel, cost_backward_kernel, gn_plus_backward_kernel, adaptive_delta_kernel,
 //   mc_epilogue_kernel, mc_lse_backward_kernel      the steps either side of the path (CTA per object).
+//   epnp_init_kernel (pnp_epnp.cuh)  EPnP initial pose of the 6DoF evaluation flow, ONE CTA per object, fp64 solve.
 // No tensor cores: the only contraction is 6-deep, the work is FP32-pipe + MUFU bound (DESIGN.md).
 // Build options: EPNP_PHASE_TIMERS (profiling), EPNP_SIMT_EMUL (g++ build for the test-only CPU emulator).
 #include <cuda_runtime.h>
@@ -20,6 +21,7 @@
 #include "pnp_device.cuh"
 #include "pnp_lm.cuh"
 #include "pnp_amis.cuh"
+#include "pnp_epnp.cuh"
 
 namespace {
 
@@ -1076,6 +1078,24 @@ int epnp_rslm_draw_f32(const float* x3d, const float* x2d, const float* w2d, con
         if (e != cudaSuccess) return cuda_fail(e);
         EPNP_LAUNCH(rslm_draw_kernel<4>, B, NT, smem, (cudaStream_t)stream, r);
     }
+    e = cudaGetLastError();
+    return e == cudaSuccess ? EPNP_OK : cuda_fail(e);
+}
+
+int epnp_epnp_init_f32(const float* x3d, const float* x2d, const float* w2d, const float* cam_mats,
+                       float conf_quantile, float* pose, int* n_used, int B, int N, void* stream) {
+    if (!x3d || !x2d || !w2d || !cam_mats || !pose || B < 0 || N <= 0) return EPNP_ERR_BAD_ARG;
+    if (!(conf_quantile >= 0.0f && conf_quantile <= 1.0f)) return EPNP_ERR_BAD_ARG;
+    if (N > EPNP_INIT_MAX_N) return EPNP_ERR_TOO_MANY_POINTS;
+    // at least N - ceil(q (N - 1)) points are >= the quantile (the virtual index as numpy computes it, in fp32)
+    const float h = conf_quantile * (float)(N - 1);
+    if (N - (int)ceilf(h) < 4) return EPNP_ERR_BAD_ARG;
+    if (B == 0) return EPNP_OK;
+    const size_t smem = (size_t)N * sizeof(float);
+    const EpnpInitArgs r{x3d, x2d, w2d, cam_mats, conf_quantile, pose, n_used, N};
+    cudaError_t e = cudaFuncSetAttribute(epnp_init_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+    if (e != cudaSuccess) return cuda_fail(e);
+    EPNP_LAUNCH(epnp_init_kernel, B, NT, smem, (cudaStream_t)stream, r);
     e = cudaGetLastError();
     return e == cudaSuccess ? EPNP_OK : cuda_fail(e);
 }

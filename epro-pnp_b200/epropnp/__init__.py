@@ -9,6 +9,7 @@ batched hot loops run in hand-written sm_100a CUDA behind libepropnp_b200.so:
     epropnp.distributions         AngularCentralGaussian / VonMisesUniformMix
     epropnp.monte_carlo_pose_loss MonteCarloPoseLoss (6DoF and detection flavours), mc_logsumexp / mc_sample_weights / mc_score_te
     epropnp.builder               build_pnp / build_camera / build_cost_fun + registries (detection-style configs)
+    epropnp.epnp_init             epnp_pose_init / EPnPSolver: the 6DoF evaluation flow's EPnP initialiser, on the device
 
 Put `<repo>/epro-pnp_b200` on sys.path (instead of the reference checkout) and existing imports keep
 working.  The solve / Monte-Carlo paths have no CPU or PyTorch fallback: CPU tensors raise.

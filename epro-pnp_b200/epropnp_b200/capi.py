@@ -46,6 +46,7 @@ _SIGNATURES = {
     "epnp_lm_solve_f32": (ctypes.c_int, [_P] * 13 + [_I, _I, ctypes.POINTER(EpnpParams), _P]),
     "epnp_gn_plus_backward_f32": (ctypes.c_int, [_P] * 13 + [_I, _I, _I, _F, _F, _F, _P]),
     "epnp_rslm_draw_f32": (ctypes.c_int, [_P] * 5 + [ctypes.c_uint64, ctypes.c_uint32, _P, _P, _P, _I, _I, _I, _I, _I, _F, _P]),
+    "epnp_epnp_init_f32": (ctypes.c_int, [_P] * 4 + [_F, _P, _P, _I, _I, _P]),
     "epnp_rslm_f32": (ctypes.c_int, [_P] * 13 + [_I, _I, _I, _I, ctypes.POINTER(EpnpParams), _P]),
     "epnp_amis_f32": (ctypes.c_int, [_P] * 12 + [ctypes.c_uint64, ctypes.c_uint32] + [_P] * 3
                       + [_I, _I, ctypes.POINTER(EpnpParams), _P]),

@@ -166,6 +166,33 @@ def rslm_draw(x3d, x2d, w2d, cam_mats, P, n, dof, eps=1e-5, seed=0, obj_offset=0
     return (inds, start, t_out) if want_t else (inds, start)
 
 
+def epnp_init(x3d, x2d, w2d, cam_mats, conf_quantile=0.8, want_count=False):
+    """EPnP initial pose per object (epnp_epnp_init_f32): the points whose confidence mean(w2d, -1) is at or above the
+    object's conf_quantile quantile (numpy 'linear'), EPnP on them in fp64.  cam_mats (3, 3) or (B, 3, 3).
+    -> pose (B, 7) = x y z w i j k with w >= 0 [, n_used (B) int32 with want_count]."""
+    _need_cuda(w2d, "w2d")
+    if x3d.dim() != 3 or x3d.shape[-1] != 3:
+        raise ValueError(f"x3d must be (B, N, 3), got {tuple(x3d.shape)}")
+    B, N = x3d.shape[0], x3d.shape[1]
+    dev = x3d.device
+    for t, shape, what in ((x2d, (B, N, 2), "x2d"), (w2d, (B, N, 2), "w2d")):
+        if tuple(t.shape) != shape or t.device != dev:
+            raise ValueError(f"{what} must be {shape} on {dev}, got {tuple(t.shape)} on {t.device}")
+    if tuple(cam_mats.shape) not in ((3, 3), (B, 3, 3)) or cam_mats.device != dev:
+        raise ValueError(f"cam_mats must be (3, 3) or ({B}, 3, 3) on {dev}, got {tuple(cam_mats.shape)}")
+    q = float(conf_quantile)
+    if not 0.0 <= q <= 1.0:
+        raise ValueError(f"conf_quantile must be in [0, 1], got {q}")
+    x3d, x2d, w2d, cam = _f32c(x3d), _f32c(x2d), _f32c(w2d), _cam(cam_mats, B, dev)
+    pose = torch.empty(B, 7, dtype=torch.float32, device=dev)
+    n_used = torch.empty(B, dtype=torch.int32, device=dev) if want_count else None
+    with torch.cuda.device(dev):
+        check(lib().epnp_epnp_init_f32(ptr(x3d), ptr(x2d), ptr(w2d), ptr(cam), ctypes.c_float(q), ptr(pose),
+                                       None if n_used is None else capi.iptr(n_used), B, N, stream_ptr(dev)),
+              "epnp_epnp_init_f32")
+    return (pose, n_used) if want_count else pose
+
+
 def rslm(prob: Problem, inds, start, params, want_all=False):
     """Fused random-sample LM initialiser (epnp_rslm_f32): inds (P, B, n) integer indices within each object, start
     (P, B, D) -> dict(pose (B, D), cost (B), pose_all (P, B, D) | None, cost_all (P, B) | None)."""
@@ -411,4 +438,4 @@ def mc_lse_backward(logw_bm, lse, grad_lse):
 
 
 __all__ = ["Problem", "adaptive_delta", "cost_backward", "evaluate_cost", "evaluate_full", "lm_solve", "amis", "lm_amis_fused",
-           "lm_amis_fused_host", "lm_amis_fused_push", "fused_workspace_bytes", "rslm", "gn_plus_backward", "mc_epilogue", "mc_lse_backward", "default_params", "NativeError", "capi"]
+           "lm_amis_fused_host", "lm_amis_fused_push", "fused_workspace_bytes", "rslm", "epnp_init", "gn_plus_backward", "mc_epilogue", "mc_lse_backward", "default_params", "NativeError", "capi"]

@@ -32,6 +32,8 @@ extern "C" {
 #endif
 
 #define EPNP_ABI_VERSION 2   /* 2: epnp_rslm_draw_f32 added; the push entry point takes DEVICE arrays of peer pointers */
+/* epnp_epnp_init_f32 was added within version 2: a new symbol, no existing one changed, so a binding written for
+ * version 2 without it keeps working. */
 
 enum {
     EPNP_OK = 0,
@@ -120,6 +122,16 @@ int epnp_rslm_draw_f32(const float* x3d, const float* x2d, const float* w2d, con
                        const float* t_init, uint64_t seed, uint32_t obj_offset,
                        int* inds, float* start, float* t_out,
                        int P, int n, int B, int N, int dof, float eps, void* stream);
+
+/* EPnP initial pose per object, as EPro-PnP-6DoF/lib/test.py:176-194 computes it with cv2.solvePnP(SOLVEPNP_EPNP):
+ *   conf[b,i] = 0.5 * (w2d[b,i,0] + w2d[b,i,1]); points with conf >= the conf_quantile quantile of the object
+ *   (numpy's default 'linear' method, evaluated in fp32 as numpy does for float32 data) are used;
+ *   pose (B, 7) = x y z w i j k with w >= 0; n_used [opt] (B) int32 = number of points used.
+ * EPnP (Lepetit, Moreno-Noguer, Fua, IJCV 2009) in pixels with fx, fy, cx, cy of cam_mats (skew ignored), fp64 inside.
+ * Rejects (EPNP_ERR_BAD_ARG) conf_quantile outside [0, 1] and N - ceil(q (N-1)) < 4;
+ * N > 16384 (a 128 x 128 map) returns EPNP_ERR_TOO_MANY_POINTS.  No lens distortion.                             */
+int epnp_epnp_init_f32(const float* x3d, const float* x2d, const float* w2d, const float* cam_mats,
+                       float conf_quantile, float* pose, int* n_used, int B, int N, void* stream);
 
 /* RSLMSolver.solve after the hypotheses are drawn (levenberg_marquardt.py:300-353): for every object, P starting
  * poses, each refined by LM / GN on its own n sampled correspondences, scored on all N correspondences, cheapest
